@@ -20,11 +20,13 @@ merge kernel.  With N > 1 the default run ALSO times that sharded step and repor
 not speed, at a size that fits one GPU -- configs[2] / configs[4] are the sizes it exists for).
 """
 import argparse
+import atexit
 import hashlib
 import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -32,7 +34,9 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
-CACHE = os.path.join(ROOT, '.index_cache')
+# codebooks and built indexes are cached outside the tree, which may be read-only
+CACHE = os.path.join(tempfile.gettempdir(), f'annlite_b200_bench_{os.getuid()}')
+DUMP_LIMIT = 64 << 20   # bytes --dump-outputs may write
 
 
 def filtered_leg(timeout_s=240):
@@ -84,7 +88,19 @@ def parse(argv=None):
     ap.add_argument('--pool', type=int, default=4, help='distinct query batches cycled through the steps')
     ap.add_argument('--no-filtered-leg', action='store_true',
                     help='skip the configs[3] side measurement (filtered search, child process, ~20 s, untimed)')
-    return ap.parse_args(argv)
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last headline step returned (rank 0) to DIR as .npy: '
+                         'labels.npy (float64, -1 = no result), distances.npy (float32) and rows.npy (the query rows '
+                         'written: all of them, or a fixed seeded sample when the batch exceeds 64 MB).  Queries, base '
+                         'vectors and codebook are the same on every run, and the index is built sequentially '
+                         '(--build-threads 1, several minutes at 1M rows) unless --build-threads says otherwise')
+    a = ap.parse_args(argv)
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
+    if a.dump_outputs and a.build_threads == 0:
+        # the concurrent builders make a different graph on every build, and two graphs share few result rows
+        a.build_threads = 1
+    return a
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -133,13 +149,15 @@ def train_codebook(a, X10k):
     if os.path.exists(p) and not a.no_cache:
         return np.load(p)
     from sklearn.cluster import KMeans
+    from threadpoolctl import threadpool_limits
     ds = a.dim // a.m
     if a.metric == 'cosine':
         X10k = X10k / np.maximum(np.linalg.norm(X10k, axis=1, keepdims=True), 1e-12)
     cb = np.empty((a.m, a.ks, ds), dtype=np.float32)
-    for m in range(a.m):
-        km = KMeans(n_clusters=a.ks, max_iter=20, n_init=1, random_state=0).fit(X10k[:, m * ds:(m + 1) * ds])
-        cb[m] = km.cluster_centers_
+    with threadpool_limits(1):   # KMeans sums in thread order: one thread gives the same codebook on every machine
+        for m in range(a.m):
+            km = KMeans(n_clusters=a.ks, max_iter=20, n_init=1, random_state=0).fit(X10k[:, m * ds:(m + 1) * ds])
+            cb[m] = km.cluster_centers_
     np.save(p, cb)
     return cb
 
@@ -158,6 +176,7 @@ class ClockSampler:
             self.p = subprocess.Popen(['nvidia-smi', f'--id={self.gpu}', f'--query-gpu={self.Q}',
                                        '--format=csv,noheader,nounits', '-lms', '20'],
                                       stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.p.kill)   # nvidia-smi -lms never exits on its own
             self.t = threading.Thread(target=self._read, daemon=True)
             self.t.start()
         except Exception:
@@ -192,6 +211,19 @@ def ncu_traffic_bytes():
         return tot or None
     except Exception:
         return None
+
+
+def dump_outputs(out_dir, labels, dists):
+    """labels (B,k) int64, dists (B,k) float32 -> out_dir/{labels,distances,rows}.npy, at most DUMP_LIMIT bytes."""
+    os.makedirs(out_dir, exist_ok=True)
+    B, k = labels.shape
+    row_bytes = k * (8 + 4) + 8
+    rows = np.arange(B)
+    if B * row_bytes > DUMP_LIMIT:
+        rows = np.sort(np.random.default_rng(0).choice(B, (DUMP_LIMIT - 4096) // row_bytes, replace=False))   # 4 KB: .npy headers
+    np.save(os.path.join(out_dir, 'labels.npy'), labels[rows].astype(np.float64))
+    np.save(os.path.join(out_dir, 'distances.npy'), dists[rows].astype(np.float32))
+    np.save(os.path.join(out_dir, 'rows.npy'), rows.astype(np.float64))
 
 
 def recall_at_k(pred, truth):
@@ -326,6 +358,8 @@ def run_ours(a):
         dist.init_process_group('nccl', device_id=torch.device('cuda', local))
     ncores = os.cpu_count() or 1
     shard_main = a.mode == 'shard' and world > 1
+    if shard_main and a.dump_outputs:
+        raise SystemExit('--dump-outputs writes the replicated step; run it without --mode shard')
 
     # ---- index: replicated on every rank (rank 0 builds, the others load the file) -----------------
     cb = train_codebook(a, make_base(a, 0, 10_000)) if rank == 0 else None
@@ -339,7 +373,7 @@ def run_ours(a):
     if a.chunks:
         e.set_option('chunks', a.chunks)
     t_build = 0.0
-    path = os.path.join(CACHE, f'ours_{cfg_key(a)}.hnsw')
+    path = os.path.join(CACHE, f'ours_{cfg_key(a, "sequential" if a.build_threads == 1 else "")}.hnsw')
     if rank == 0:
         t_build = _build_or_load(a, e, 0, a.n, path, a.build_threads)   # 0 threads = library default (<= 32, quota-aware)
     if world > 1:
@@ -394,6 +428,8 @@ def run_ours(a):
         clocks.start()
         time.sleep(0.05)
     ms, launches = _timed(torch, dist, e, world, step_dev_stream, a.steps, a.warmup, drain)
+    last = (a.warmup + a.steps - 1) & 1                                      # step i wrote out_l2[i & 1]
+    last_step = (out_l2[last].cpu().numpy(), out_d2[last].cpu().numpy()) if a.dump_outputs else None
     ms_e2e, _ = _timed(torch, dist, e, world, step_e2e_stream, a.steps, max(3, a.warmup // 2), drain)
     ms_sync, _ = _timed(torch, dist, e, world, step_dev, a.steps, 3)            # one blocking call per step, for reference
     ms_e2e_sync, _ = _timed(torch, dist, e, world, step_e2e, a.steps, 3)
@@ -529,6 +565,8 @@ def run_ours(a):
         dist.barrier()
         dist.destroy_process_group()
     if rank == 0:
+        if last_step is not None:
+            dump_outputs(a.dump_outputs, *last_step)
         print(json.dumps(result))
 
 
